@@ -12,6 +12,7 @@ PAF line scoring -> per-edge assignment -> greedy grouping (-> all_gather of ins
 
 Prints ONE JSON line (rank 0).  `value` = frames/s with frames resident in HBM; `e2e` = the same
 metric through the public `predict_on_batch` call with pinned host frames (H2D + D2H inside).
+Frames and weights are seeded, so `--dump-outputs DIR` gives the same inputs' results from any build.
 """
 import argparse
 import json
@@ -339,6 +340,27 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def dump_outputs(out_dir, records, max_instances, n_nodes):
+    """Writes the results of the last timed step as ``out_dir/<name>.npy`` (float32): the per-frame records the grouping
+    kernel left on the device, split into the arrays ``predict_on_batch`` returns for the same frames.
+
+    Those arrays hold NaN in instance slots past ``n_valid``, for nodes an instance lacks and for peaks whose refinement
+    failed.  Every file written here is finite: each of the three result arrays is stored with 0 in place of those
+    entries, next to ``<name>_finite.npy`` (1 where the library returned a finite value, 0 where it returned NaN)."""
+    from sleap_b200 import parallel
+    rec = records.cpu()
+    peaks, vals, scores, n_valid = parallel.unpack_records(rec, max_instances, n_nodes)
+    flags = rec[:, max_instances * n_nodes * 3 + max_instances + 1]
+    out = {"n_valid": n_valid.numpy(), "flags": flags.numpy()}
+    for name, a in (("instance_peaks", peaks), ("instance_peak_vals", vals), ("instance_scores", scores)):
+        a = a.numpy()
+        finite = np.isfinite(a)
+        out[name], out[name + "_finite"] = np.where(finite, a, 0.0), finite
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
+
 # --------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -368,11 +390,12 @@ def run_ours(args):
     spec = c4_spec()
     cm = A.compile_model(spec, 1)
     weights = A.make_synthetic_weights(cm, SEED)
+    # calibrated on the fp32 CPU oracle network, as the reference arm is: the head weights are an input of the benchmark
+    # and must not depend on the build under test or on the conv variants its autotuner picks in this run
+    from oracle import convnet, preprocess as opre
     calib = make_frames(2, 500)
-    m0 = DeviceModel(spec, weights, input_channels=1, precision=prec, handle=handle)
-    cms0, pafs0 = m0.forward(calib)
+    cms0, pafs0 = convnet.model_forward(opre.preprocess(calib, True, 1.0, 32), spec, weights)
     weights = calibrate_heads(weights, cms0, pafs0, len(calib))
-    del m0
     model = DeviceModel(spec, weights, input_channels=1, precision=prec, handle=handle)
     pred = BottomUpPredictor(model, NODES, EDGES, peak_threshold=0.2, batch_size=B, integral_refinement=True,
                              max_peaks_per_sample=1024, max_node_peaks=32, max_instances_per_frame=32)
@@ -482,6 +505,8 @@ def run_ours(args):
         ev1.record(stream)
     barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, t_rec, I, C)
     fwd_ms = np.zeros(max(args.steps, 1), np.float32)
     n_fwd = c_int32(0)
     handle.call("sb_model_forward_times", model.model_id, 0, len(fwd_ms), _lib.ptr(fwd_ms), byref(n_fwd))
@@ -728,7 +753,12 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the (untimed) fp16-vs-fp32 parity block")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ncu-step", action="store_true", help="profiler window (cudaProfilerStart/Stop) around --steps warm steps, no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results (rank 0's frames) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
     # keep stdout clean for the ONE JSON line (NCCL / torchrun print banners on stdout)
     saved_stdout = os.dup(1)
     os.dup2(2, 1)

@@ -16,9 +16,11 @@ Outputs:
   models/<name>/fixture_config.json    the training config reduced to the keys the inference path reads
   models/<name>/best_model.npz         float32 weights {layer/param} read out of best_model.h5 (optimizer state dropped)
   frames_minimal_instance.npz, frames_robot.npz   uint8 frames + ground-truth points (frame, instance, node, xy)
+  h5py/<path under tests/data>         files written by h5py, for the in-tree HDF5 reader and writer tests (H5PY_FILES)
 """
 import json
 import os
+import shutil
 import sys
 
 import cv2
@@ -39,6 +41,33 @@ MODELS = {
     "min_tracks_2node.bottomup_multiclass": "min_tracks_2node.UNet.bottomup_multiclass",
     "min_tracks_2node.topdown_multiclass": "min_tracks_2node.UNet.topdown_multiclass",
 }
+
+
+H5PY_FILES = ["slp_hdf5/minimal_instance.slp", "slp_hdf5/small_robot_minimal.slp", "slp_hdf5/dance.mp4.labels.slp",
+              "models/minimal_robot.UNet.single_instance/best_model.h5"]
+
+
+def copy_h5py_files():
+    """Byte-for-byte copies, except that the data of every ``optimizer_weights`` dataset of a ``best_model.h5`` (the Adam
+    state, 60 % of the file, which inference never reads) is overwritten with zeros so that the stored file compresses.
+    The HDF5 structure, the model weights and every other byte stay as h5py wrote them."""
+    for rel in H5PY_FILES:
+        src, dst = os.path.join(REF, rel), os.path.join(HERE, "h5py", rel)
+        os.makedirs(os.path.dirname(dst), exist_ok=True)
+        if not rel.endswith(".h5"):
+            shutil.copyfile(src, dst)
+            continue
+        f = h5lite.File(src)
+        r = f._r
+        buf = bytearray(r.b)
+        for _, ds in f["optimizer_weights"].visit_datasets():
+            for t, _, p, _ in r.messages(ds._addr):
+                if t == 0x08:                                  # data layout message, version 3, contiguous storage
+                    assert r.b[p] == 3 and r.b[p + 1] == 1, rel
+                    a, n = r.u64(p + 2), r.u64(p + 10)
+                    buf[a:a + n] = bytes(n)
+        with open(dst, "wb") as out:
+            out.write(buf)
 
 
 def reduced_config(cfg):
@@ -131,6 +160,8 @@ def main():
     np.savez_compressed(os.path.join(HERE, "frames_tracks_2node.npz"), images=frames, points_gt=np.stack(rows)[None], frame_idx=np.asarray(idxs),
                         track_names=np.asarray(gt_tracks(slp, 1)), video_json=np.asarray(json.dumps(vid)))
     print("tracks_2node", frames.shape, np.stack(rows).shape, idxs, gt_tracks(slp, 1), vid)
+
+    copy_h5py_files()
 
 
 if __name__ == "__main__":

@@ -33,13 +33,9 @@ def frames(name):
     return z["images"], z["points_gt"]
 
 
-REF_DATA = "/root/reference/tests/data"       # present in the build container only; never read by the -m gpu tests
-
-
-def ref_path(*parts):
-    """A data file of the reference checkout, or None where the checkout does not exist (GPU box)."""
-    p = os.path.join(REF_DATA, *parts)
-    return p if os.path.exists(p) else None
+def h5py_file(*parts):
+    """A file of the reference's test data that h5py wrote, stored under tests/golden/h5py/ by its path in that data."""
+    return os.path.join(GOLDEN, "h5py", *parts)
 
 
 def labels_minimal_instance():

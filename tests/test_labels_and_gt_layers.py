@@ -9,12 +9,9 @@ from sleap_b200.io.labels import Labels, LabelsReader, Skeleton, find_instance_c
 from sleap_b200.io.video import Video
 from sleap_b200.nn.inference import FindInstancePeaksGroundTruth
 
-import pytest
-
 import reference_models as rm
 
-REF_SLP = rm.ref_path("slp_hdf5", "minimal_instance.slp")
-needs_reference = pytest.mark.skipif(REF_SLP is None, reason="reads h5py-written files of the reference checkout")
+REF_SLP = rm.h5py_file("slp_hdf5", "minimal_instance.slp")
 
 
 def _labels():
@@ -22,7 +19,6 @@ def _labels():
     return rm.labels_minimal_instance(), z
 
 
-@needs_reference
 def test_labels_load_file():
     lab = Labels.load_file(REF_SLP)
     z = np.load(os.path.join(rm.GOLDEN, "frames_minimal_instance.npz"))
@@ -31,9 +27,9 @@ def test_labels_load_file():
     assert lab.video_specs[0]["backend"]["grayscale"] is True
     assert_allclose(np.stack([i.numpy() for i in lab[0].instances]), z["points_gt"][0], rtol=1e-6)
     assert lab[0][0].n_visible_points == 2 and not lab[0][0].predicted
-    robot = Labels.load_file(rm.ref_path("slp_hdf5", "small_robot_minimal.slp"))
+    robot = Labels.load_file(rm.h5py_file("slp_hdf5", "small_robot_minimal.slp"))
     assert [lf.frame_idx for lf in robot] == [0, 79] and len(robot[1]) == 1
-    dance = Labels.load_file(rm.ref_path("slp_hdf5", "dance.mp4.labels.slp"))
+    dance = Labels.load_file(rm.h5py_file("slp_hdf5", "dance.mp4.labels.slp"))
     assert len(dance) == 450 and len(dance.skeleton) == 17 and len(dance.skeleton.edge_names) == 15
     assert sum(len(lf.predicted_instances) for lf in dance) == 450 and sum(len(lf.user_instances) for lf in dance) == 3
     # the rebuilt fixture used by the GPU tests equals what the file holds

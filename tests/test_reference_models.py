@@ -6,7 +6,6 @@ Also exercises the in-tree HDF5 reader on the committed Keras .h5 / .slp files."
 import os
 
 import numpy as np
-import pytest
 from numpy.testing import assert_allclose
 
 from oracle import inference as oinf
@@ -19,12 +18,10 @@ def _matched(points_gt, points_pr, atol):
     assert_allclose(points_gt[i1], points_pr[i2], atol=atol)
 
 
-REF_H5 = rm.ref_path("models", "minimal_robot.UNet.single_instance", "best_model.h5")
-REF_SLP = rm.ref_path("slp_hdf5", "minimal_instance.slp")
-needs_reference = pytest.mark.skipif(REF_H5 is None or REF_SLP is None, reason="reads h5py-written files of the reference checkout")
+REF_H5 = rm.h5py_file("models", "minimal_robot.UNet.single_instance", "best_model.h5")
+REF_SLP = rm.h5py_file("slp_hdf5", "minimal_instance.slp")
 
 
-@needs_reference
 def test_h5_reader_keras_weights_match_npz_export():
     """The in-tree HDF5 reader on a Keras ``best_model.h5`` written by h5py: every array equals the committed ``.npz``."""
     from sleap_b200.io import h5lite
@@ -44,7 +41,6 @@ def test_h5_reader_keras_weights_match_npz_export():
             np.testing.assert_array_equal(a, wz[layer][k])
 
 
-@needs_reference
 def test_h5_reader_slp_tables():
     from sleap_b200.io import h5lite
     f = h5lite.File(REF_SLP)
@@ -58,11 +54,9 @@ def test_h5_reader_slp_tables():
     assert f["metadata"].attrs["format_id"] == 1.1 or str(f["metadata"].attrs["format_id"]).startswith("1.1")
     _, gt = rm.frames("minimal_instance")
     assert_allclose(gt[0, 0, 0], [pts["x"][0], pts["y"][0]], rtol=1e-6)
-    big = rm.ref_path("slp_hdf5", "dance.mp4.labels.slp")                       # chunked tables, 450 frames of predictions
-    if big:
-        g = h5lite.File(big)
-        assert g["frames"].read().shape == (450,) and g["pred_points"].read().shape == (7650,)
-        assert g["instances"].read().dtype.names[-1] == "tracking_score"
+    g = h5lite.File(rm.h5py_file("slp_hdf5", "dance.mp4.labels.slp"))          # chunked tables, 450 frames of predictions
+    assert g["frames"].read().shape == (450,) and g["pred_points"].read().shape == (7650,)
+    assert g["instances"].read().dtype.names[-1] == "tracking_score"
 
 
 def test_oracle_bottomup_on_trained_model():

@@ -11,12 +11,9 @@ from numpy.testing import assert_array_equal
 from sleap_b200.io import h5lite, h5write
 from sleap_b200.io import labels as L
 
-import pytest
-
 import reference_models as rm
 
-GOLDEN = rm.ref_path("slp_hdf5", "minimal_instance.slp")          # written by h5py (reference checkout, build container only)
-needs_reference = pytest.mark.skipif(GOLDEN is None, reason="compares with h5py-written files of the reference checkout")
+GOLDEN = rm.h5py_file("slp_hdf5", "minimal_instance.slp")          # written by h5py
 
 
 def _messages(path, name):
@@ -26,7 +23,6 @@ def _messages(path, name):
     return r, {t: r.b[p:p + sz] for t, fl, p, sz in r.messages(addr)}
 
 
-@needs_reference
 def test_datatype_and_dataspace_messages_match_h5py_bytes():
     legacy_instance = np.dtype([(n, L.INSTANCE_DTYPE.fields[n][0]) for n in L.INSTANCE_DTYPE.names[:-1]])   # fixture predates tracking_score
     for name, dt in (("frames", L.FRAME_DTYPE), ("instances", legacy_instance), ("points", L.POINT_DTYPE),
@@ -43,7 +39,6 @@ def test_datatype_and_dataspace_messages_match_h5py_bytes():
     assert msgs[0x0003][:20] == h5write.encode_datatype(np.dtype("f8"))
 
 
-@needs_reference
 def test_superblock_and_group_structures_match_h5py(tmp_path):
     p = str(tmp_path / "w.slp")
     with h5write.File(p) as f:
